@@ -17,6 +17,12 @@ In frames mode the line also carries `shard_selfcheck` (max |err| of one sharded
 unsharded on the same GPU) and `exchange` (device time of the separable exchange launches of one UNet forward).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--stage 1|2] [--shard videos|frames] [--impl reference]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (the decoded frames of rank 0's video) as DIR/frames.npy,
+float32: whole when it fits in 64 MB (stage 1: 16 x 3 x 512 x 512), else a fixed sample (stage 2, see `dump_outputs`).
+Inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.  The
+GroupNorm statistics are accumulated with float atomics, so two runs agree to rounding, not bit for bit.
 
 stdout carries exactly one line, the JSON (libraries that print to fd 1 are redirected to stderr).  Keys beyond the
 contract: `unet_ms_per_sampler_step` (one eager UNet forward with the host kept ahead of the GPU = the cost of a sampler
@@ -341,9 +347,34 @@ def unet_step_flops(stage: int, latent: int) -> float:
     return fl
 
 
+DUMP_BYTES = 64 * 10 ** 6      # all of what --dump-outputs writes
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes each array as <out_dir>/<name>.npy in float32.  One whose float32 size exceeds its share of DUMP_BYTES is
+    written as a fixed sample instead: the flattened array at the first k indices of
+    numpy.random.RandomState(0).permutation(numel), sorted (a 1-D array; RandomState keeps its stream across numpy
+    versions)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.float().numpy()
+        what = f"{a.shape}"
+        if a.nbytes > share:
+            k = (share - 4096) // 4                    # leave room for the .npy header
+            idx = np.sort(np.random.RandomState(0).permutation(a.size)[:k])
+            a = a.reshape(-1)[idx]
+            what = f"a fixed sample of {k} of the {t.numel()} elements of {tuple(t.shape)}"
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        print(f"[bench] --dump-outputs: {name}.npy = {what}", file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------------------------------------------
-def measure(model, stage, engine, rank, world, local, dev, steps, warmup, frames_mode, dist, want_breakdown, peaks):
-    """Warm up, time `steps` videos device-resident and e2e; returns a dict of raw results (rank 0 has everything)."""
+def measure(model, stage, engine, rank, world, local, dev, steps, warmup, frames_mode, dist, want_breakdown, peaks,
+            keep_output=False):
+    """Warm up, time `steps` videos device-resident and e2e; returns a dict of raw results (rank 0 has everything).
+    keep_output: also return what the last timed resident step computed, on the host (`output`)."""
     import torch
     from hi3d_official_b200 import _native
     wl = workload(stage)
@@ -376,8 +407,12 @@ def measure(model, stage, engine, rank, world, local, dev, steps, warmup, frames
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item()), _native.launch_count() - l0
 
+    last = [None]
+
     def step_resident():
-        run_video(model, stage, dev_t, shard)
+        out = run_video(model, stage, dev_t, shard)
+        if keep_output:
+            last[0] = out
 
     def step_e2e():
         d = {k: v.to(dev, non_blocking=True) for k, v in host.items()}
@@ -392,9 +427,11 @@ def measure(model, stage, engine, rank, world, local, dev, steps, warmup, frames
         clocks.start()
     ms, launches = timed(step_resident, steps)
     clk = clocks.stop() if rank == 0 else None
+    output = last[0].cpu() if keep_output else None      # before the e2e steps can reuse its memory
     step_e2e()
     ms_e2e, _ = timed(step_e2e, steps)
-    res = dict(ms=ms, ms_e2e=ms_e2e, launches=launches, clocks=clk, h2d=h2d, d2h=d2h, breakdown=None, roof=None, unet_ms=None)
+    res = dict(ms=ms, ms_e2e=ms_e2e, launches=launches, clocks=clk, h2d=h2d, d2h=d2h, breakdown=None, roof=None, unet_ms=None,
+               output=output)
     if rank == 0 and want_breakdown and not frames_mode:
         res["breakdown"], res["roof"], res["unet_ms"] = kernel_breakdown(model, stage, dev_t, peaks)
     if frames_mode:
@@ -514,7 +551,13 @@ def main():
     ap.add_argument("--ref-latent", type=int, default=0,
                     help="TESTS ONLY (--impl reference): latent size override so the CPU suite finishes in seconds; the line "
                          "then says so in config.reference_latent_override and is not a bench value")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path, not --impl reference")
     # stdout carries exactly ONE line, the JSON: anything a library writes to fd 1 in between (NCCL prints its version
     # banner there) goes to stderr instead
     sys.stdout.flush()
@@ -564,7 +607,9 @@ def main():
 
     model = build(args.stage)
     r = measure(model, args.stage, args.engine, rank, world, local, dev, args.steps, args.warmup, frames_mode, dist,
-                not args.no_breakdown, peaks)
+                not args.no_breakdown, peaks, keep_output=bool(args.dump_outputs) and rank == 0)
+    if r["output"] is not None:
+        dump_outputs(args.dump_outputs, {"frames": r.pop("output")})
     stage1 = None
     if rank == 0 and world == 1 and args.stage == 2 and not args.no_stage1:
         del model

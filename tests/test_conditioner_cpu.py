@@ -1,5 +1,6 @@
 """SURVEY §8f N2: the conditioner pieces that need no third-party weights, against the unmodified reference classes
-(where /root/reference is importable) and against their definitions."""
+(their outputs and the reference's inference-v02 config, stored under tests/golden/ by `tools/make_golden.py
+--only-parity`) and against their definitions."""
 import os
 
 import pytest
@@ -7,31 +8,28 @@ import torch
 
 from hi3d_official_b200 import conditioner as Cn
 from hi3d_official_b200 import util
-from oracle import ref_import as R
 
-needs_ref = pytest.mark.skipif(not R.available(), reason="reference tree absent")
+G = os.path.join(os.path.dirname(__file__), "golden")
 
 
-@needs_ref
+def _golden():
+    return torch.load(os.path.join(G, "conditioner.pt"), weights_only=False)
+
+
 def test_concat_timestep_embedder_matches_reference():
-    R.setup()
-    from sgm.modules.encoders.modules import ConcatTimestepEmbedderND as Ref
-    g = torch.Generator().manual_seed(0)
-    for x in (torch.rand(3, generator=g) * 30, torch.rand(2, 3, generator=g) * 5, torch.tensor([0.02])):
-        torch.testing.assert_close(Cn.ConcatTimestepEmbedderND(256)(x), Ref(256)(x), rtol=1e-5, atol=1e-5)
+    for x, ref in _golden()["timestep_embedder"]:
+        torch.testing.assert_close(Cn.ConcatTimestepEmbedderND(256)(x), ref, rtol=1e-5, atol=1e-5)
 
 
-@needs_ref
 def test_video_prediction_embedder_arrangement_matches_reference():
     """Frame / copy bookkeeping of VideoPredictionEmbedderWithEncoder (modules.py:1012-1021) with an identity 'encoder'."""
-    R.setup()
-    from sgm.modules.encoders.modules import VideoPredictionEmbedderWithEncoder as Ref
     cfg = {"target": "torch.nn.Identity"}
+    fix = _golden()["video_prediction"]
     vid = torch.arange(2 * 3 * 4 * 5 * 5, dtype=torch.float32).reshape(6, 4, 5, 5)      # (b t) = 2 x 3 cond frames
+    assert torch.equal(vid, fix["vid"])
     for ncf, ncp in ((3, 1), (1, 4), (3, 2)):
         mine = Cn.VideoPredictionEmbedderWithEncoder(ncf, ncp, cfg, scale_factor=0.5)
-        ref = Ref(n_cond_frames=ncf, n_copies=ncp, encoder_config=cfg, scale_factor=0.5, disable_encoder_autocast=True)
-        torch.testing.assert_close(mine(vid.clone()), ref(vid.clone()))
+        torch.testing.assert_close(mine(vid.clone()), fix["out"][(ncf, ncp)])
 
 
 def test_depth_pixel_unshuffle_and_normalisation():
@@ -65,12 +63,11 @@ def test_clip_embedder_bookkeeping_and_aes_vector():
     assert a.preprocess(x).shape == (2, 3, 224, 224)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/configs/inference-v02.yaml"), reason="reference configs absent")
 def test_unmodified_conditioner_config_produces_reference_shaped_conditioning():
-    """The conditioner_config of the UNMODIFIED inference-v02.yaml, with the towers' outputs supplied in the batch and a
-    stub in place of the VAE encoder: keys, shapes, concat order [depth 9 | latent 4], vector = [elevation | cond_aug],
-    and the force_uc_zero_embeddings semantics of pipeline_i2v_eval_v02.py:111-118."""
-    cfg = util.load_yaml("/root/reference/configs/inference-v02.yaml")["model"]["params"]["conditioner_config"]
+    """The conditioner_config of the UNMODIFIED inference-v02.yaml (stored parsed, as JSON), with the towers' outputs
+    supplied in the batch and a stub in place of the VAE encoder: keys, shapes, concat order [depth 9 | latent 4],
+    vector = [elevation | cond_aug], and the force_uc_zero_embeddings semantics of pipeline_i2v_eval_v02.py:111-118."""
+    cfg = util.load_yaml(os.path.join(G, "inference-v02.json"))["model"]["params"]["conditioner_config"]
     with torch.device("meta"):
         cond = util.instantiate_from_config(cfg)
     names = [type(e).__name__ for e in cond.embedders]

@@ -149,12 +149,12 @@ def test_config_glue_resolves_reference_targets_and_builds_on_meta():
     assert float(uc["crossattn"].abs().sum()) == 0 and float(uc["concat"].abs().sum()) == 0 and torch.equal(uc["vector"], c["vector"])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/configs/inference-v01.yaml"), reason="reference configs absent")
 @pytest.mark.parametrize("name,adm,cin", [("inference-v01.yaml", 768, 8), ("inference-v02.yaml", 512, 17)])
 def test_unmodified_reference_yaml_instantiates(name, adm, cin):
+    """The reference's inference configs, stored parsed (JSON is YAML) under tests/golden/ by tools/make_golden.py."""
     from hi3d_official_b200 import engine
     with torch.device("meta"):
-        m = engine.create_model(f"/root/reference/configs/{name}")
+        m = engine.create_model(os.path.join(ROOT, "tests", "golden", name.replace(".yaml", ".json")))
     u = m.model.diffusion_model
     assert u.cfg.adm_in_channels == adm and u.in_channels == cin and m.en_and_decode_n_samples_a_time in (1, 16)
     assert type(m).__name__ in ("VideoLDM", "VideoLDMStage2")
@@ -193,7 +193,7 @@ def test_flop_count_matches_survey():
 
 
 def test_bench_reference_arm_prints_one_json_line():
-    """`bench.py --impl reference` (the CPU arm the driver times): exactly one stdout line, the contract's keys."""
+    """`bench.py --impl reference` (the CPU arm): exactly one stdout line with the keys every bench line carries."""
     import json
     import os
     import subprocess
@@ -208,8 +208,11 @@ def test_bench_reference_arm_prints_one_json_line():
     for k in ("impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
               "vs_baseline", "dtype", "data", "config", "cpu_baseline", "e2e"):
         assert k in d, k
-    # the unmodified reference modules (/root/reference here, their staged copy oracle/_ref on the GPU box), not the port
-    assert d["impl"] == "reference" and d["value"] > 0 and d["cpu_baseline"]["kind"] == "reference"
+    # the unmodified reference modules wherever they can be imported (the reference tree, or the copy oracle/build_ref.py
+    # staged under oracle/_ref); without them the arm times the oracle port and says so
+    from oracle import ref_import as R
+    assert d["impl"] == "reference" and d["value"] > 0
+    assert d["cpu_baseline"]["kind"] == ("reference" if R.available() else "port")
     assert d["config"]["reference_latent_override"] == 8 and d["sampler_steps_timed"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert "workload" in d["config"]
