@@ -50,6 +50,8 @@ _SIGS = {
     "hi3d_gemm": (C.c_int, [C.POINTER(GemmParams), C.c_void_p]),
     "hi3d_gemm_tc5": (C.c_int, [C.POINTER(GemmParams), C.c_void_p]),
     "hi3d_gemm_tc5_set_pair_mode": (C.c_int, [C.c_int]),
+    "hi3d_gemm_det": (C.c_int, [C.POINTER(GemmParams), C.c_void_p, C.c_int64, C.c_void_p]),
+    "hi3d_gemm_tc5_det": (C.c_int, [C.POINTER(GemmParams), C.c_void_p, C.c_int64, C.c_void_p]),
     "hi3d_gemm_tc5_set_epilogue_warps": (C.c_int, [C.c_int]),
     "hi3d_groupnorm_ws_floats": (C.c_int64, [C.c_int]),
     "hi3d_groupnorm_silu": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_void_p,
@@ -68,6 +70,16 @@ _SIGS = {
     "hi3d_groupnorm_apply_halo": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_int64,
                                             C.c_void_p, C.c_void_p, C.c_float, C.c_int, C.c_void_p, C.c_int64, C.c_int64,
                                             C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "hi3d_groupnorm_silu_det": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_void_p,
+                                          C.c_void_p, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "hi3d_groupnorm_sums_det": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_void_p,
+                                          C.c_void_p, C.c_void_p]),
+    "hi3d_groupnorm_group_sums_det": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                C.c_void_p, C.c_void_p]),
+    "hi3d_groupnorm_unit_stats_det": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
+                                                C.c_int64, C.c_void_p]),
+    "hi3d_groupnorm_partials_floats": (C.c_int64, [C.c_int, C.c_int64, C.c_int, C.c_int]),
+    "hi3d_groupnorm_fold": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "hi3d_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p,
                                  C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
     "hi3d_attention_d64": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_void_p]),

@@ -352,7 +352,8 @@ int validate_gemm(const hi3d_gemm_params* p, const char* who) {
 
 using namespace hi3d;
 
-extern "C" int hi3d_gemm(const hi3d_gemm_params* p, void* stream) {
+// partials != NULL: deterministic GroupNorm statistics (hi3d_gemm_det)
+static int gemm_mma(const hi3d_gemm_params* p, float* partials, int64_t partials_floats, void* stream) {
   int rc = validate_gemm(p, "hi3d_gemm");
   if (rc) return rc;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -379,8 +380,18 @@ extern "C" int hi3d_gemm(const hi3d_gemm_params* p, void* stream) {
     return -2;
   }
   if (p->out_up && !(p->out_py == 1 && p->out_px == 1)) return 0;
+  if (partials != nullptr)
+    return hi3d_groupnorm_unit_stats_det(p->out, p->N, p->M / p->gn_rows, (int64_t)p->gn_rows * (p->out_up ? 4 : 1), p->gn_unit,
+                                         p->gn_stats, partials, partials_floats, stream);
   return hi3d_groupnorm_unit_stats(p->out, p->N, p->M / p->gn_rows, (int64_t)p->gn_rows * (p->out_up ? 4 : 1), p->gn_unit,
                                    p->gn_stats, stream);
+}
+
+extern "C" int hi3d_gemm(const hi3d_gemm_params* p, void* stream) { return gemm_mma(p, nullptr, 0, stream); }
+
+extern "C" int hi3d_gemm_det(const hi3d_gemm_params* p, float* partials, int64_t partials_floats, void* stream) {
+  if (!partials) { set_error("hi3d_gemm_det: null partials table"); return -2; }
+  return gemm_mma(p, partials, partials_floats, stream);
 }
 
 extern "C" const char* hi3d_last_error(void) { return hi3d::g_err; }

@@ -70,6 +70,9 @@ struct T5Params {
   float* gn_stats;
   int gn_unit, gn_rows, gn_units, gn_nimg;   // channels per unit, GEMM-grid rows per image, units per image (N / unit), images
   int gelu_poly;                             // GEGLU gate: 1 = MUFU-free polynomial erf (gelu_poly2), 0 = Abramowitz-Stegun form
+  // deterministic statistics (EPI_*_GN_DET): slot table [image][parity class][32-row block of the image][octet][4]
+  float* gn_part;
+  int gn_bpi;                                // 32-row blocks per image and parity class (gn_rows / 32)
 };
 
 // gelu(x) = 0.5 x (1 + erf(x / sqrt 2)) with erf from Abramowitz-Stegun 7.1.26 (|err| < 1.5e-7 + MUFU error, far
@@ -195,7 +198,10 @@ HI3D_DEVINL long long t5_map(const T5Params& p, long long m) {
 // kernel parameter) was profiled at 12 % instruction-cache misses and 6 % branch stalls on the short-K GEMMs, whose epilogue
 // IS the kernel (ncu source page, profiles/r02_ncu_gemm_epilogue_notes.txt): the options that cost code and branches inside the
 // chunk loop -- GEGLU, residual, blend, GroupNorm statistics -- are template constants in the specialised kernels.
-enum { EPI_GENERIC = 0, EPI_GEGLU = 1, EPI_BIAS = 2, EPI_RES = 3, EPI_RESBLEND = 4, EPI_BIAS_GN = 5, EPI_RES_GN = 6, EPI_RESBLEND_GN = 7 };
+// The *_GN_DET variants store the statistics partials into per-warp slots instead of adding them with RED (deterministic mode,
+// hi3d_gemm_tc5_det): separate instantiations, so that the default ones keep their registers and code.
+enum { EPI_GENERIC = 0, EPI_GEGLU = 1, EPI_BIAS = 2, EPI_RES = 3, EPI_RESBLEND = 4, EPI_BIAS_GN = 5, EPI_RES_GN = 6, EPI_RESBLEND_GN = 7,
+       EPI_BIAS_GN_DET = 8, EPI_RES_GN_DET = 9, EPI_RESBLEND_GN_DET = 10 };
 
 // EW = epilogue warps (8 or 16).  Sixteen (four per TMEM lane quarter, every fourth 32-column chunk each) double the
 // epilogue's issue slots and loads / stores in flight for the short-K GEMMs whose epilogue is the bound; the register-light
@@ -205,8 +211,10 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tc5_kernel(const __grid_
   constexpr bool kGen = (EPI == EPI_GENERIC);
   // compile-time constants in the specialised kernels, run-time tests in the generic one
   const bool kGeglu = kGen ? (p.act == HI3D_ACT_GEGLU) : (EPI == EPI_GEGLU);
-  const bool kRes = kGen ? (p.residual != nullptr) : (EPI == EPI_RES || EPI == EPI_RESBLEND || EPI == EPI_RES_GN || EPI == EPI_RESBLEND_GN);
-  const bool kBlend = kGen ? (p.blend_x != nullptr) : (EPI == EPI_RESBLEND || EPI == EPI_RESBLEND_GN);
+  const bool kRes = kGen ? (p.residual != nullptr) : (EPI == EPI_RES || EPI == EPI_RESBLEND || EPI == EPI_RES_GN || EPI == EPI_RESBLEND_GN ||
+                                                      EPI == EPI_RES_GN_DET || EPI == EPI_RESBLEND_GN_DET);
+  const bool kBlend = kGen ? (p.blend_x != nullptr) : (EPI == EPI_RESBLEND || EPI == EPI_RESBLEND_GN || EPI == EPI_RESBLEND_GN_DET);
+  constexpr bool kDet = (EPI >= EPI_BIAS_GN_DET);
   const bool kSilu = kGen ? (p.act == HI3D_ACT_SILU) : false;
   const bool kGn = kGen ? (p.gn_stats != nullptr && p.act != HI3D_ACT_GEGLU) : (EPI >= EPI_BIAS_GN);
   const int kDbg = kGen ? p.dbg : 0;
@@ -406,6 +414,22 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tc5_kernel(const __grid_
 #pragma unroll
         for (int i = 0; i < 4; i++) gn_srow[i] = __shfl_sync(0xffffffffu, sl, crow + 8 * i);
       }
+      // deterministic mode: this warp's slot row = (image, parity class, block of the image).  The host takes this path only
+      // when every warp block lies inside one image: PLAIN gn_rows % 32 == 0, CONV2D tw * th >= 32, TEMPORAL ts >= 32.
+      float* gn_slot = nullptr;
+      if (kDet && gn_wsmp >= 0) {
+        int loc;
+        if (p.mode == HI3D_ROWS_PLAIN) {
+          loc = (int)((((long long)mt * T5_BM + q * 32) % p.gn_rows) / 32);
+        } else {
+          // blocks of one image inside a tile: CONV2D a tw x th patch, TEMPORAL ts = tw pixels of one frame
+          const int bpf = ((p.mode == HI3D_ROWS_CONV2D) ? p.tw * p.th : p.tw) / 32;
+          const int tx = mt % p.tiles_x, ty = (mt / p.tiles_x) % p.tiles_y;
+          loc = (p.mode == HI3D_ROWS_CONV2D) ? (ty * p.tiles_x + tx) * bpf + q % bpf : tx * bpf + q % bpf;
+        }
+        const int npar = p.out_up ? 4 : 1, par = p.out_up ? 2 * p.out_py + p.out_px : 0;
+        gn_slot = p.gn_part + ((long long)((gn_s0 + gn_wsmp) * npar + par) * p.gn_bpi + loc) * (long long)(p.N / 2);
+      }
       const __half* rbp = nullptr;
       if (p.rowbias != nullptr && m >= 0) rbp = p.rowbias + (long long)((m / p.rb_div) % p.rb_mod) * p.rb_ld;
       const uint32_t buf = at & 1;
@@ -536,7 +560,7 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tc5_kernel(const __grid_
             // flushed once per tile -- shared float atomics are compare-and-swap loops and the flush needed a 256-thread
             // barrier per tile; it cost the GEMMs more than the statistics pass it replaced.)
             const int cbase = n + cchk * 8;
-            if (gn_uniform && p.gn_unit >= 4) {
+            if (kDet || (gn_uniform && p.gn_unit >= 4)) {
               float2 s2[4], q2[4];                 // packed fp32: channel pairs (2k, 2k+1) summed over this lane's rows
 #pragma unroll
               for (int k = 0; k < 4; k++) s2[k] = q2[k] = make_float2(0.f, 0.f);
@@ -567,7 +591,11 @@ __global__ void __launch_bounds__(64 + 32 * EW, 1) gemm_tc5_kernel(const __grid_
                 sA += __shfl_xor_sync(0xffffffffu, sA, off); qA += __shfl_xor_sync(0xffffffffu, qA, off);
                 sB += __shfl_xor_sync(0xffffffffu, sB, off); qB += __shfl_xor_sync(0xffffffffu, qB, off);
               }
-              if (lane < 4 && gn_wsmp >= 0 && colok) {
+              if (kDet) {
+                // slot (warp block, octet): written by exactly one lane of one warp, read by hi3d_groupnorm_fold
+                if (lane < 4 && gn_slot != nullptr && colok)
+                  *reinterpret_cast<float4*>(gn_slot + (cbase / 8) * 4) = make_float4(sA, qA, sB, qB);
+              } else if (lane < 4 && gn_wsmp >= 0 && colok) {
                 float* dst = p.gn_stats + ((long long)(gn_s0 + gn_wsmp) * p.gn_units + ua) * 2;
                 atomicAdd(dst, sA); atomicAdd(dst + 1, qA);                       // results unused -> RED
                 if (nb < 8 && ua + 1 < p.gn_units) { atomicAdd(dst + 2, sB); atomicAdd(dst + 3, qB); }
@@ -702,6 +730,9 @@ static int launch_tc5_n(int epi, int ew, const T5Params& tp, int smem, int smem_
     case EPI_BIAS_GN: return launch_tc5_one<NCTA, EPI_BIAS_GN, 8>(tp, smem, smem_total, units, sm_count, st);
     case EPI_RES_GN: return launch_tc5_one<NCTA, EPI_RES_GN, 8>(tp, smem, smem_total, units, sm_count, st);
     case EPI_RESBLEND_GN: return launch_tc5_one<NCTA, EPI_RESBLEND_GN, 8>(tp, smem, smem_total, units, sm_count, st);
+    case EPI_BIAS_GN_DET: return launch_tc5_one<NCTA, EPI_BIAS_GN_DET, 8>(tp, smem, smem_total, units, sm_count, st);
+    case EPI_RES_GN_DET: return launch_tc5_one<NCTA, EPI_RES_GN_DET, 8>(tp, smem, smem_total, units, sm_count, st);
+    case EPI_RESBLEND_GN_DET: return launch_tc5_one<NCTA, EPI_RESBLEND_GN_DET, 8>(tp, smem, smem_total, units, sm_count, st);
     default: return launch_tc5_one<NCTA, EPI_GENERIC, 8>(tp, smem, smem_total, units, sm_count, st);
   }
 }
@@ -730,9 +761,12 @@ extern "C" int hi3d_gemm_tc5_set_epilogue_warps(int warps) {
   return 0;
 }
 
-extern "C" int hi3d_gemm_tc5(const hi3d_gemm_params* p, void* stream) {
+// partials != NULL: deterministic GroupNorm statistics (hi3d_gemm_tc5_det); geometries this engine does not cover go to
+// hi3d_gemm / hi3d_gemm_det accordingly
+static int gemm_tc5(const hi3d_gemm_params* p, float* partials, int64_t partials_floats, void* stream) {
   int rc = validate_gemm(p, "hi3d_gemm_tc5");
   if (rc) return rc;
+  auto fallback = [&]() { return partials ? hi3d_gemm_det(p, partials, partials_floats, stream) : hi3d_gemm(p, stream); };
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   // ---- geometry this engine covers; everything else goes to the mma.sync engine (same results) ----
   T5Params tp;
@@ -787,7 +821,7 @@ extern "C" int hi3d_gemm_tc5(const hi3d_gemm_params* p, void* stream) {
     tp.seg[i].map = mi; tp.seg[i].c_off = s.c_off; tp.seg[i].C = s.C;
     tp.seg[i].dy = s.dy; tp.seg[i].dx = s.dx; tp.seg[i].dt = s.dt;
   }
-  if (!ok) return hi3d_gemm(p, stream);
+  if (!ok) return fallback();
 
   // tile-N: multiple of 32 in [32, 256].  Cost model = rounds of the persistent grid x time per tile, where a tile
   // costs its MMA columns plus a fixed term (A-operand traffic / epilogue set-up); this accounts both for the padding
@@ -828,14 +862,35 @@ extern "C" int hi3d_gemm_tc5(const hi3d_gemm_params* p, void* stream) {
     tp.gn_units = p->N / p->gn_unit; tp.gn_nimg = p->M / p->gn_rows;
   }
   tp.gelu_poly = g_gelu_poly;
+  // deterministic statistics (hi3d_gemm_tc5_det): per-warp slots from the specialised epilogues when every 32-row
+  // warp block lies inside one image and an octet reaches into at most two units; otherwise no epilogue statistics and a
+  // deterministic statistics pass over the stored tensor after the launch
+  const bool has_res = p->residual != nullptr, has_blend = p->blend_x != nullptr;
+  const bool det = p->gn_stats != nullptr && partials != nullptr;
+  const int det_npar = p->out_up ? 4 : 1;
+  bool det_slots = false;
+  if (det) {
+    const bool one_image = (p->mode == HI3D_ROWS_PLAIN) ? (p->gn_rows % 32 == 0)
+                           : (p->mode == HI3D_ROWS_CONV2D) ? (tp.tw * tp.th >= 32) : (tp.tw >= 32);
+    det_slots = one_image && (p->gn_unit == 4 || p->gn_unit >= 8) && g_dbg == 0 && p->act == HI3D_ACT_NONE &&
+                !(has_blend && !has_res);
+    const int64_t need = det_slots ? (int64_t)tp.gn_nimg * det_npar * (p->gn_rows / 32) * (p->N / 8) * 4 : 0;
+    if (partials_floats < need || (!det_slots && p->out_ld != p->N)) {
+      set_error("hi3d_gemm_tc5: deterministic statistics need %lld partials floats (have %lld) and out_ld == N (%d, %d)",
+                (long long)need, (long long)partials_floats, p->out_ld, p->N);
+      return -2;
+    }
+    if (det_slots) { tp.gn_part = partials; tp.gn_bpi = p->gn_rows / 32; }
+    else tp.gn_stats = nullptr;
+  }
+  const bool has_gn = tp.gn_stats != nullptr;
   // epilogue specialisation and epilogue warp count (decided here: the scratch of 16 warps comes out of the stage budget)
   int epi = EPI_GENERIC;
-  const bool has_res = p->residual != nullptr, has_blend = p->blend_x != nullptr, has_gn = p->gn_stats != nullptr;
   if (g_dbg == 0 && p->act != HI3D_ACT_SILU && !(has_blend && !has_res)) {
     if (p->act == HI3D_ACT_GEGLU) epi = (has_res || has_blend || has_gn) ? EPI_GENERIC : EPI_GEGLU;
-    else if (has_blend) epi = has_gn ? EPI_RESBLEND_GN : EPI_RESBLEND;
-    else if (has_res) epi = has_gn ? EPI_RES_GN : EPI_RES;
-    else epi = has_gn ? EPI_BIAS_GN : EPI_BIAS;
+    else if (has_blend) epi = has_gn ? (det_slots ? EPI_RESBLEND_GN_DET : EPI_RESBLEND_GN) : EPI_RESBLEND;
+    else if (has_res) epi = has_gn ? (det_slots ? EPI_RES_GN_DET : EPI_RES_GN) : EPI_RES;
+    else epi = has_gn ? (det_slots ? EPI_BIAS_GN_DET : EPI_BIAS_GN) : EPI_BIAS;
   }
   // 16 epilogue warps when the epilogue is the bound: short K (main loop of a tile shorter than its epilogue)
   int ew = 8;
@@ -844,7 +899,7 @@ extern "C" int hi3d_gemm_tc5(const hi3d_gemm_params* p, void* stream) {
   const int stage_bytes = T5_A_BYTES + (BN / ncta) * 128;
   int stages = (T5_SMEM_BUDGET - gn_tab_bytes - extra_scr) / stage_bytes;
   if (stages > T5_MAX_STAGES) stages = T5_MAX_STAGES;
-  if (stages < 2) { return hi3d_gemm(p, stream); }
+  if (stages < 2) { return fallback(); }
   tp.BN = BN; tp.stages = stages;
   tp.n_tiles = (p->N + BN - 1) / BN;
   tp.total_tiles = m_units * tp.n_tiles;      // (pair-)tiles
@@ -887,5 +942,18 @@ extern "C" int hi3d_gemm_tc5(const hi3d_gemm_params* p, void* stream) {
   const int smem = stages * stage_bytes + 16 * T5_MAX_STAGES + 64 + 2048 + ew * T5_SCR_BYTES + gn_tab_bytes + 1024;
   rc = launch_tc5(ncta, epi, ew, tp, smem, smem_total, units, g_sm_count, st);
   if (rc) return rc;
-  return check_launch("hi3d_gemm_tc5");
+  rc = check_launch("hi3d_gemm_tc5");
+  // deterministic statistics: fold the slots (or run the pass) once the tensor is complete -- after the last parity launch
+  if (rc || !det || (p->out_up && !(p->out_py == 1 && p->out_px == 1))) return rc;
+  if (det_slots)
+    return hi3d_groupnorm_fold(partials, tp.gn_nimg, det_npar * (p->gn_rows / 32), 1, p->N, p->gn_unit, p->gn_stats, stream);
+  return hi3d_groupnorm_unit_stats_det(p->out, p->N, tp.gn_nimg, (int64_t)p->gn_rows * det_npar, p->gn_unit, p->gn_stats,
+                                       partials, partials_floats, stream);
+}
+
+extern "C" int hi3d_gemm_tc5(const hi3d_gemm_params* p, void* stream) { return gemm_tc5(p, nullptr, 0, stream); }
+
+extern "C" int hi3d_gemm_tc5_det(const hi3d_gemm_params* p, float* partials, int64_t partials_floats, void* stream) {
+  if (!partials) { set_error("hi3d_gemm_tc5_det: null partials table"); return -2; }
+  return gemm_tc5(p, partials, partials_floats, stream);
 }

@@ -24,6 +24,9 @@ HI3D_DEVINL Half8 ld_stream(const __half* p) {
 
 // ---- pass 1: per-(sample, chunk, group) partial sum / sum of squares -------------------------------
 // grid (chunks, n_samples); blockDim = RL * CV where CV = C/8 vector-columns.
+// DET: the per-CTA group sums are formed in a fixed order (per-thread channel sums staged in shared memory, then one thread per
+// (group, sum | sumsq) adds them channel-major, row-lane-minor) instead of shared-memory float atomics.
+template <bool DET>
 __global__ void __launch_bounds__(512)
 gn_stats_kernel(const __half* __restrict__ x1, int C1, const __half* __restrict__ x2, int C2, long long rows_per_sample,
                 long long rows_per_chunk, float* __restrict__ ws) {
@@ -68,6 +71,20 @@ gn_stats_kernel(const __half* __restrict__ x1, int C1, const __half* __restrict_
       s[2 * k + 1] += f.y; q[2 * k + 1] += f.y * f.y;
     }
   }
+  if constexpr (DET) {
+    __shared__ float sch[2][512 * 8];           // [s | q][rl * C + channel]
+#pragma unroll
+    for (int e = 0; e < 8; e++) { sch[0][rl * C + c0 + e] = s[e]; sch[1][rl * C + c0 + e] = q[e]; }
+    __syncthreads();
+    if (tid < GN_GROUPS * 2) {
+      const int g = tid >> 1, which = tid & 1;
+      float acc = 0.f;
+      for (int c = g * cpg; c < (g + 1) * cpg; c++)
+        for (int l = 0; l < RL; l++) acc += sch[which][l * C + c];
+      ws[((long long)n * GN_MAX_CHUNKS + chunk) * (GN_GROUPS * 2) + tid] = acc;
+    }
+    return;
+  }
   // fold the 8 channels into their groups (a vector may straddle a group boundary when cpg % 8 != 0)
   int gcur = c0 / cpg;
   float as = 0.f, aq = 0.f;
@@ -87,6 +104,8 @@ gn_stats_kernel(const __half* __restrict__ x1, int C1, const __half* __restrict_
 
 // ---- pass 1b: combine the chunk partials of one sample into (sum, sum of squares) per group ----------------
 // grid (n_samples), 1024 threads; result at fin[n][32][2].  (Frame-sharded runs all-reduce `fin` across ranks here.)
+// DET: the 16 per-thread partials of a value are added in thread order instead of with shared-memory atomics.
+template <bool DET>
 __global__ void __launch_bounds__(1024)
 gn_finalize_kernel(const float* __restrict__ ws, int nchunks, float* __restrict__ fin) {
   __shared__ float stot[GN_GROUPS * 2];
@@ -104,6 +123,17 @@ gn_finalize_kernel(const float* __restrict__ ws, int nchunks, float* __restrict_
     a3 += w[(c + 48) * (GN_GROUPS * 2) + (tid & 63)];
   }
   for (; c < nchunks; c += 16) a0 += w[c * (GN_GROUPS * 2) + (tid & 63)];
+  if constexpr (DET) {
+    __shared__ float spart[16][GN_GROUPS * 2];
+    spart[tid >> 6][tid & 63] = (a0 + a1) + (a2 + a3);
+    __syncthreads();
+    if (tid < GN_GROUPS * 2) {
+      float acc = 0.f;
+      for (int k = 0; k < 16; k++) acc += spart[k][tid];
+      fin[(long long)n * (GN_GROUPS * 2) + tid] = acc;
+    }
+    return;
+  }
   atomicAdd(&stot[tid & 63], (a0 + a1) + (a2 + a3));
   __syncthreads();
   if (tid < GN_GROUPS * 2) fin[(long long)n * (GN_GROUPS * 2) + tid] = stot[tid];
@@ -377,8 +407,9 @@ static int gn_check(const void* x1, int C1, const void* x2, int C2, int n_sample
 }
 
 // (sum, sum of squares) per (sample, group) of the LOCAL rows -> sums[n_samples][32][2] (fp32)
-extern "C" int hi3d_groupnorm_sums(const void* x1, int C1, const void* x2, int C2, int n_samples, int64_t rows_per_sample,
-                                   float* sums, float* ws, void* stream) {
+template <bool DET>
+static int groupnorm_sums(const void* x1, int C1, const void* x2, int C2, int n_samples, int64_t rows_per_sample, float* sums,
+                          float* ws, void* stream) {
   if (!x2) C2 = 0;
   int rc = gn_check(x1, C1, x2, C2, n_samples, rows_per_sample, "hi3d_groupnorm_sums");
   if (rc) return rc;
@@ -396,12 +427,22 @@ extern "C" int hi3d_groupnorm_sums(const void* x1, int C1, const void* x2, int C
   long long rpc = (rows_per_sample + chunks - 1) / chunks;
   rpc = (rpc + RL - 1) / RL * RL;
   chunks = (rows_per_sample + rpc - 1) / rpc;
-  gn_stats_kernel<<<dim3((unsigned)chunks, n_samples), threads, 0, st>>>((const __half*)x1, C1, (const __half*)x2, C2,
+  gn_stats_kernel<DET><<<dim3((unsigned)chunks, n_samples), threads, 0, st>>>((const __half*)x1, C1, (const __half*)x2, C2,
                                                                         rows_per_sample, rpc, ws);
   rc = check_launch("hi3d_groupnorm_sums(stats)");
   if (rc) return rc;
-  gn_finalize_kernel<<<n_samples, 1024, 0, st>>>(ws, (int)chunks, sums);
+  gn_finalize_kernel<DET><<<n_samples, 1024, 0, st>>>(ws, (int)chunks, sums);
   return check_launch("hi3d_groupnorm_sums(finalize)");
+}
+
+extern "C" int hi3d_groupnorm_sums(const void* x1, int C1, const void* x2, int C2, int n_samples, int64_t rows_per_sample,
+                                   float* sums, float* ws, void* stream) {
+  return groupnorm_sums<false>(x1, C1, x2, C2, n_samples, rows_per_sample, sums, ws, stream);
+}
+
+extern "C" int hi3d_groupnorm_sums_det(const void* x1, int C1, const void* x2, int C2, int n_samples, int64_t rows_per_sample,
+                                       float* sums, float* ws, void* stream) {
+  return groupnorm_sums<true>(x1, C1, x2, C2, n_samples, rows_per_sample, sums, ws, stream);
 }
 
 // hi3d_groupnorm_apply_stats routes through the same launcher; its extra arguments travel in these thread-locals
@@ -471,7 +512,10 @@ extern "C" int hi3d_groupnorm_apply_halo(const void* x1, int C1, const void* x2,
 
 // ---- unit statistics of an existing tensor: (sum, sumsq) per image and per `unit` consecutive channels, accumulated -------
 // grid (chunks, n_images); same streaming pattern as gn_stats_kernel, folding into units instead of the 32 groups.
+// DET: no atomics -- the CTA's unit sums are formed in a fixed order (as in gn_stats_kernel<true>) and STORED into its own
+// partials slot, stats = fp32 [n_images, chunks, units, 2]; gn_fold_kernel then sums the slots of an image in chunk order.
 constexpr int GN_MAX_UNITS = 256;
+template <bool DET>
 __global__ void __launch_bounds__(512)
 gn_unit_stats_kernel(const __half* __restrict__ x, int C, long long rows_per_image, long long rows_per_chunk, int unit,
                      float* __restrict__ stats) {
@@ -514,6 +558,21 @@ gn_unit_stats_kernel(const __half* __restrict__ x, int C, long long rows_per_ima
       s[2 * k + 1] += f.y; q[2 * k + 1] += f.y * f.y;
     }
   }
+  if constexpr (DET) {
+    __shared__ float sch[2][512 * 8];           // [s | q][rl * C + channel]
+#pragma unroll
+    for (int e = 0; e < 8; e++) { sch[0][rl * C + c0 + e] = s[e]; sch[1][rl * C + c0 + e] = q[e]; }
+    __syncthreads();
+    float* slot = stats + ((long long)n * gridDim.x + blockIdx.x) * nu * 2;
+    for (int i = tid; i < nu * 2; i += blockDim.x) {
+      const int u = i >> 1, which = i & 1;
+      float acc = 0.f;
+      for (int c = u * unit; c < (u + 1) * unit; c++)
+        for (int l = 0; l < RL; l++) acc += sch[which][l * C + c];
+      slot[i] = acc;
+    }
+    return;
+  }
   int ucur = c0 / unit;
   float as = 0.f, aq = 0.f;
 #pragma unroll
@@ -531,11 +590,29 @@ gn_unit_stats_kernel(const __half* __restrict__ x, int C, long long rows_per_ima
 }
 
 // unit tables -> (sum, sumsq) per (sample, group): sums[n][32][2]
+// DET: one thread per (group, sum | sumsq) adds its table entries image-major, unit-minor (the order of the gn_apply prologue).
+template <bool DET>
 __global__ void __launch_bounds__(256)
 gn_group_sums_kernel(const float* __restrict__ stats1, int C1, const float* __restrict__ stats2, int C2, int unit, int ips,
                      float* __restrict__ sums) {
   __shared__ float ssum[GN_GROUPS * 2];
   const int tid = threadIdx.x, n = blockIdx.x;
+  if constexpr (DET) {
+    if (tid < GN_GROUPS * 2) {
+      const int g = tid >> 1, which = tid & 1;
+      const int upg = (C1 + C2) / GN_GROUPS / unit, u1 = C1 / unit, u2 = C2 / unit;
+      float acc = 0.f;
+      for (int img = 0; img < ips; img++) {
+        const long long im = (long long)n * ips + img;
+        for (int uu = 0; uu < upg; uu++) {
+          const int u = g * upg + uu;
+          acc += (u < u1) ? stats1[(im * u1 + u) * 2 + which] : stats2[(im * u2 + (u - u1)) * 2 + which];
+        }
+      }
+      sums[(long long)n * (GN_GROUPS * 2) + tid] = acc;
+    }
+    return;
+  }
   if (tid < GN_GROUPS * 2) ssum[tid] = 0.f;
   __syncthreads();
   const int cpg = (C1 + C2) / GN_GROUPS, upg = cpg / unit, u1 = C1 / unit, u2 = C2 / unit;
@@ -553,6 +630,47 @@ gn_group_sums_kernel(const float* __restrict__ stats1, int C1, const float* __re
   if (tid < GN_GROUPS * 2) sums[(long long)n * (GN_GROUPS * 2) + tid] = ssum[tid];
 }
 
+// ---- fold: partials table -> unit table [n_images, units, 2], OVERWRITTEN --------------------------------------------------
+// grid (units, n_images), GN_FOLD_THREADS threads.  Thread t adds the slots t, t + GN_FOLD_THREADS, ... in fp64, then a fixed
+// shared-memory tree combines the threads: the order depends on the shapes only.  Two slot layouts:
+//   octets = 0: [n_images][nblk][units][2]            (gn_unit_stats_kernel<true>: one slot per (image, chunk))
+//   octets = 1: [n_images][nblk][C / 8][4]             (gemm_tc5 deterministic epilogue: one slot per (image, 32-row block,
+//               8-channel octet) = (sum, sumsq) of the octet's first unit, then of the next unit it reaches into (unit >= 4))
+constexpr int GN_FOLD_THREADS = 128;
+__global__ void __launch_bounds__(GN_FOLD_THREADS)
+gn_fold_kernel(const float* __restrict__ part, int nblk, int octets, int C, int unit, float* __restrict__ stats) {
+  __shared__ double red[2][GN_FOLD_THREADS];
+  const int u = blockIdx.x, n = blockIdx.y, nu = C / unit, tid = threadIdx.x;
+  double as = 0.0, aq = 0.0;
+  if (octets) {
+    const int noct = C / 8, o0 = (u * unit) / 8, o1 = ((u + 1) * unit - 1) / 8;
+    const float* base = part + (long long)n * nblk * noct * 4;
+    for (int b = tid; b < nblk; b += GN_FOLD_THREADS)
+      for (int o = o0; o <= o1; o++) {
+        const int side = ((o * 8) / unit == u) ? 0 : 2;     // the octet's first unit, or the one after it
+        const float2 v = *reinterpret_cast<const float2*>(base + ((long long)b * noct + o) * 4 + side);
+        as += (double)v.x; aq += (double)v.y;
+      }
+  } else {
+    const float* base = part + (long long)n * nblk * nu * 2 + u * 2;
+    for (int b = tid; b < nblk; b += GN_FOLD_THREADS) {
+      as += (double)base[(long long)b * nu * 2];
+      aq += (double)base[(long long)b * nu * 2 + 1];
+    }
+  }
+  red[0][tid] = as; red[1][tid] = aq;
+  __syncthreads();
+#pragma unroll
+  for (int h = GN_FOLD_THREADS / 2; h > 0; h >>= 1) {
+    if (tid < h) { red[0][tid] += red[0][tid + h]; red[1][tid] += red[1][tid + h]; }
+    __syncthreads();
+  }
+  if (tid == 0) {
+    stats[((long long)n * nu + u) * 2] = (float)red[0][0];
+    stats[((long long)n * nu + u) * 2 + 1] = (float)red[1][0];
+  }
+}
+
 static int unit_check(int C1, int C2, int unit, const char* who) {
   const int C = C1 + C2;
   if (unit <= 0 || (C % GN_GROUPS) || ((C / GN_GROUPS) % unit) || (C1 % unit) || (C2 % unit) || C1 / unit > GN_MAX_UNITS ||
@@ -564,13 +682,8 @@ static int unit_check(int C1, int C2, int unit, const char* who) {
   return 0;
 }
 
-extern "C" int hi3d_groupnorm_unit_stats(const void* x, int C, int n_images, int64_t rows_per_image, int unit, float* stats,
-                                         void* stream) {
-  if (!x || !stats || C <= 0 || (C % 8) || n_images <= 0 || n_images > 65535 || rows_per_image <= 0 || unit <= 0 ||
-      (C % unit) || C / unit > GN_MAX_UNITS || ((uintptr_t)x & 15)) {
-    set_error("hi3d_groupnorm_unit_stats: bad arguments (C=%d unit=%d n=%d rows=%lld)", C, unit, n_images, (long long)rows_per_image);
-    return -2;
-  }
+// grid of gn_unit_stats_kernel: `chunks` CTAs of `threads` per image, rpc rows each
+static long long unit_stats_grid(int C, int n_images, int64_t rows_per_image, int* threads_out, long long* rpc_out) {
   const int CV = C / 8;
   const int threads = (512 / CV) * CV;
   const int RL = threads / CV;
@@ -581,19 +694,93 @@ extern "C" int hi3d_groupnorm_unit_stats(const void* x, int C, int n_images, int
   long long rpc = (rows_per_image + chunks - 1) / chunks;
   rpc = (rpc + RL - 1) / RL * RL;
   chunks = (rows_per_image + rpc - 1) / rpc;
-  gn_unit_stats_kernel<<<dim3((unsigned)chunks, n_images), threads, 0, (cudaStream_t)stream>>>((const __half*)x, C, rows_per_image,
+  *threads_out = threads;
+  *rpc_out = rpc;
+  return chunks;
+}
+
+static int unit_stats_args(const void* x, int C, int n_images, int64_t rows_per_image, int unit, const float* stats,
+                           const char* who) {
+  if (!x || !stats || C <= 0 || (C % 8) || n_images <= 0 || n_images > 65535 || rows_per_image <= 0 || unit <= 0 ||
+      (C % unit) || C / unit > GN_MAX_UNITS || ((uintptr_t)x & 15)) {
+    set_error("%s: bad arguments (C=%d unit=%d n=%d rows=%lld)", who, C, unit, n_images, (long long)rows_per_image);
+    return -2;
+  }
+  return 0;
+}
+
+extern "C" int hi3d_groupnorm_unit_stats(const void* x, int C, int n_images, int64_t rows_per_image, int unit, float* stats,
+                                         void* stream) {
+  int rc = unit_stats_args(x, C, n_images, rows_per_image, unit, stats, "hi3d_groupnorm_unit_stats");
+  if (rc) return rc;
+  int threads;
+  long long rpc;
+  const long long chunks = unit_stats_grid(C, n_images, rows_per_image, &threads, &rpc);
+  gn_unit_stats_kernel<false><<<dim3((unsigned)chunks, n_images), threads, 0, (cudaStream_t)stream>>>((const __half*)x, C, rows_per_image,
                                                                                               rpc, unit, stats);
   return check_launch("hi3d_groupnorm_unit_stats");
 }
 
-extern "C" int hi3d_groupnorm_group_sums(const float* stats1, int C1, const float* stats2, int C2, int unit, int n_samples,
-                                         int imgs_per_sample, float* sums, void* stream) {
+extern "C" int64_t hi3d_groupnorm_partials_floats(int n_images, int64_t rows_per_image, int C, int unit) {
+  if (n_images <= 0 || rows_per_image <= 0 || C <= 0 || (C % 8) || unit <= 0 || (C % unit)) return 0;
+  int threads;
+  long long rpc;
+  const long long chunks = unit_stats_grid(C, n_images, rows_per_image, &threads, &rpc);
+  const int64_t pass = (int64_t)n_images * chunks * (C / unit) * 2;                    // gn_unit_stats_kernel<true>
+  const int64_t epi = (int64_t)n_images * ((rows_per_image + 31) / 32) * (C / 8) * 4;   // gemm_tc5 deterministic epilogue
+  return pass > epi ? pass : epi;
+}
+
+extern "C" int hi3d_groupnorm_fold(const float* partials, int n_images, int blocks_per_image, int octets, int C, int unit,
+                                   float* stats, void* stream) {
+  if (!partials || !stats || n_images <= 0 || n_images > 65535 || blocks_per_image <= 0 || C <= 0 || (C % 8) || unit <= 0 ||
+      (C % unit) || C / unit > GN_MAX_UNITS || (octets && unit < 4)) {
+    set_error("hi3d_groupnorm_fold: bad arguments (n=%d blocks=%d C=%d unit=%d)", n_images, blocks_per_image, C, unit);
+    return -2;
+  }
+  gn_fold_kernel<<<dim3((unsigned)(C / unit), n_images), GN_FOLD_THREADS, 0, (cudaStream_t)stream>>>(
+      partials, blocks_per_image, octets ? 1 : 0, C, unit, stats);
+  return check_launch("hi3d_groupnorm_fold");
+}
+
+extern "C" int hi3d_groupnorm_unit_stats_det(const void* x, int C, int n_images, int64_t rows_per_image, int unit, float* stats,
+                                             float* partials, int64_t partials_floats, void* stream) {
+  int rc = unit_stats_args(x, C, n_images, rows_per_image, unit, stats, "hi3d_groupnorm_unit_stats_det");
+  if (rc) return rc;
+  int threads;
+  long long rpc;
+  const long long chunks = unit_stats_grid(C, n_images, rows_per_image, &threads, &rpc);
+  if (!partials || partials_floats < (int64_t)n_images * chunks * (C / unit) * 2) {
+    set_error("hi3d_groupnorm_unit_stats_det: partials table of %lld floats, %lld needed", (long long)partials_floats,
+              (long long)n_images * chunks * (C / unit) * 2);
+    return -2;
+  }
+  gn_unit_stats_kernel<true><<<dim3((unsigned)chunks, n_images), threads, 0, (cudaStream_t)stream>>>((const __half*)x, C,
+                                                                                             rows_per_image, rpc, unit, partials);
+  rc = check_launch("hi3d_groupnorm_unit_stats_det");
+  if (rc) return rc;
+  return hi3d_groupnorm_fold(partials, n_images, (int)chunks, 0, C, unit, stats, stream);
+}
+
+template <bool DET>
+static int group_sums(const float* stats1, int C1, const float* stats2, int C2, int unit, int n_samples, int imgs_per_sample,
+                      float* sums, void* stream) {
   if (!stats2) C2 = 0;
   if (!stats1 || !sums || n_samples <= 0 || imgs_per_sample <= 0) { set_error("hi3d_groupnorm_group_sums: bad arguments"); return -2; }
   int rc = unit_check(C1, C2, unit, "hi3d_groupnorm_group_sums");
   if (rc) return rc;
-  gn_group_sums_kernel<<<n_samples, 256, 0, (cudaStream_t)stream>>>(stats1, C1, stats2, C2, unit, imgs_per_sample, sums);
+  gn_group_sums_kernel<DET><<<n_samples, 256, 0, (cudaStream_t)stream>>>(stats1, C1, stats2, C2, unit, imgs_per_sample, sums);
   return check_launch("hi3d_groupnorm_group_sums");
+}
+
+extern "C" int hi3d_groupnorm_group_sums(const float* stats1, int C1, const float* stats2, int C2, int unit, int n_samples,
+                                         int imgs_per_sample, float* sums, void* stream) {
+  return group_sums<false>(stats1, C1, stats2, C2, unit, n_samples, imgs_per_sample, sums, stream);
+}
+
+extern "C" int hi3d_groupnorm_group_sums_det(const float* stats1, int C1, const float* stats2, int C2, int unit, int n_samples,
+                                             int imgs_per_sample, float* sums, void* stream) {
+  return group_sums<true>(stats1, C1, stats2, C2, unit, n_samples, imgs_per_sample, sums, stream);
 }
 
 extern "C" int hi3d_groupnorm_apply_stats(const void* x1, int C1, const float* stats1, const void* x2, int C2, const float* stats2,
@@ -612,15 +799,27 @@ extern "C" int hi3d_groupnorm_apply_stats(const void* x1, int C1, const float* s
   return rc;
 }
 
-extern "C" int hi3d_groupnorm_silu(const void* x1, int C1, const void* x2, int C2, int n_samples,
-                                   int64_t rows_per_sample, const float* gamma, const float* beta, float eps,
-                                   int apply_silu, void* y, float* ws, void* stream) {
+template <bool DET>
+static int groupnorm_silu(const void* x1, int C1, const void* x2, int C2, int n_samples, int64_t rows_per_sample,
+                          const float* gamma, const float* beta, float eps, int apply_silu, void* y, float* ws, void* stream) {
   if (!ws) { set_error("hi3d_groupnorm_silu: null workspace"); return -2; }
   float* sums = ws + (long long)n_samples * GN_MAX_CHUNKS * GN_GROUPS * 2;
-  int rc = hi3d_groupnorm_sums(x1, C1, x2, C2, n_samples, rows_per_sample, sums, ws, stream);
+  int rc = groupnorm_sums<DET>(x1, C1, x2, C2, n_samples, rows_per_sample, sums, ws, stream);
   if (rc) return rc;
   return hi3d_groupnorm_apply(x1, C1, x2, C2, n_samples, rows_per_sample, sums, rows_per_sample, gamma, beta, eps, apply_silu,
                               y, 0, 0, stream);
+}
+
+extern "C" int hi3d_groupnorm_silu(const void* x1, int C1, const void* x2, int C2, int n_samples,
+                                   int64_t rows_per_sample, const float* gamma, const float* beta, float eps,
+                                   int apply_silu, void* y, float* ws, void* stream) {
+  return groupnorm_silu<false>(x1, C1, x2, C2, n_samples, rows_per_sample, gamma, beta, eps, apply_silu, y, ws, stream);
+}
+
+extern "C" int hi3d_groupnorm_silu_det(const void* x1, int C1, const void* x2, int C2, int n_samples,
+                                       int64_t rows_per_sample, const float* gamma, const float* beta, float eps,
+                                       int apply_silu, void* y, float* ws, void* stream) {
+  return groupnorm_silu<true>(x1, C1, x2, C2, n_samples, rows_per_sample, gamma, beta, eps, apply_silu, y, ws, stream);
 }
 
 extern "C" int hi3d_layernorm(const void* x, const void* addvec, int add_div, int add_mod, int64_t M, int C,

@@ -58,9 +58,19 @@ def gather_to_rank0(x: torch.Tensor) -> Optional[torch.Tensor]:
 # Used by the launch plan (unet._Plan) when HI3D_SHARD_EXCHANGE=nccl; the default on B200 is the peer-memory form
 # (peer.py + the sharded kernels), which needs no collective library on the step's path.  These operate in place on the
 # plan's own buffers and are backend-agnostic, so tests/test_dist_cpu.py runs exactly this code under 2-rank gloo.
-def allreduce_sum_(t: torch.Tensor) -> torch.Tensor:
-    """[B, 32, 2] (sum, sumsq) GroupNorm partials of this rank's frames -> totals over all frames of the clip."""
-    if world()[1] > 1:
+def allreduce_sum_(t: torch.Tensor, deterministic: bool = False) -> torch.Tensor:
+    """[B, 32, 2] (sum, sumsq) GroupNorm partials of this rank's frames -> totals over all frames of the clip.
+    deterministic: an all-gather and a sum in rank order (the order of the peer-memory exchange kernel), so that every rank
+    gets the same bits run after run; an NCCL all-reduce picks its own reduction order."""
+    ws = world()[1]
+    if ws > 1 and deterministic:
+        parts = [torch.empty_like(t) for _ in range(ws)]
+        dist.all_gather(parts, t.contiguous())
+        acc = parts[0].clone()
+        for p in parts[1:]:
+            acc += p
+        t.copy_(acc)
+    elif ws > 1:
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
     return t
 

@@ -7,6 +7,7 @@ replayed step costs one ctypes call per launch.
 from __future__ import annotations
 
 import ctypes as C
+import os
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -15,6 +16,13 @@ from . import _native as N
 from ._native import ACT_GEGLU, ACT_NONE, ACT_SILU, ROWS_CONV2D, ROWS_PLAIN, ROWS_TEMPORAL  # noqa: F401
 
 F16 = torch.float16
+
+
+def deterministic() -> bool:
+    """The deterministic-mode switch, read when a launch plan is built (and part of its key): GroupNorm statistics without
+    float atomics, so that the same inputs give bit-identical outputs.  On with torch.use_deterministic_algorithms(True) or
+    HI3D_DETERMINISTIC=1 (for jobs that cannot change code, e.g. torchrun / bench.py)."""
+    return torch.are_deterministic_algorithms_enabled() or os.environ.get("HI3D_DETERMINISTIC") == "1"
 
 
 def _stream() -> int:
@@ -71,7 +79,8 @@ class Gemm:
                  geom: Optional[dict] = None, bias: Optional[torch.Tensor] = None,
                  rowbias: Optional[torch.Tensor] = None, rb_div: int = 1, rb_mod: int = 1, act: int = ACT_NONE,
                  residual: Optional[torch.Tensor] = None, blend_x: Optional[torch.Tensor] = None, alpha: float = 0.0,
-                 engine: str = "mma", gn_stats: Optional[torch.Tensor] = None, gn_unit: int = 0, gn_rows: int = 0):
+                 engine: str = "mma", gn_stats: Optional[torch.Tensor] = None, gn_unit: int = 0, gn_rows: int = 0,
+                 gn_partials: Optional[torch.Tensor] = None):
         _chk16(W, "W")
         _chk16(out, "out")
         Nn, K = W.shape
@@ -120,13 +129,20 @@ class Gemm:
                 raise ValueError(f"gn_stats: unit {gn_unit} / rows {gn_rows} do not fit N={Nn}, M={M}, table {tuple(gn_stats.shape)}")
             p.gn_stats, p.gn_unit, p.gn_rows = gn_stats.data_ptr(), gn_unit, gn_rows
         self.p = p
-        self._keep = (list(segs), W, out, bias, rowbias, residual, blend_x, gn_stats)   # keep storages alive
-        self._fn = N.load().hi3d_gemm_tc5 if engine == "tc5" else N.load().hi3d_gemm
+        self._keep = (list(segs), W, out, bias, rowbias, residual, blend_x, gn_stats, gn_partials)   # keep storages alive
+        self._det = ()
+        if gn_stats is not None and gn_partials is not None:
+            # deterministic statistics (hi3d_gemm_det / hi3d_gemm_tc5_det): gn_stats is overwritten, gn_partials is scratch
+            _chk32(gn_partials, "gn_partials")
+            self._det = (gn_partials.data_ptr(), gn_partials.numel())
+            self._fn = N.load().hi3d_gemm_tc5_det if engine == "tc5" else N.load().hi3d_gemm_det
+        else:
+            self._fn = N.load().hi3d_gemm_tc5 if engine == "tc5" else N.load().hi3d_gemm
         self.flops = 2.0 * M * Nn * K
         self.out = out
 
     def __call__(self):
-        rc = self._fn(C.byref(self.p), _stream())
+        rc = self._fn(C.byref(self.p), *self._det, _stream())
         if rc:
             N.check(rc, "hi3d_gemm")
 
@@ -138,23 +154,25 @@ def groupnorm_ws(n_samples: int, device) -> torch.Tensor:
 
 def groupnorm_silu(x1: torch.Tensor, x2: Optional[torch.Tensor], n_samples: int, rows_per_sample: int,
                    gamma: torch.Tensor, beta: torch.Tensor, eps: float, silu: bool, y: torch.Tensor,
-                   ws: torch.Tensor):
+                   ws: torch.Tensor, det: bool = False):
     _chk16(x1, "x1"); _chk16(y, "y"); _chk32(gamma, "gamma"); _chk32(beta, "beta")
     c2 = 0
     if x2 is not None:
         _chk16(x2, "x2")
         c2 = x2.shape[-1]
-    N.check(N.load().hi3d_groupnorm_silu(x1.data_ptr(), x1.shape[-1], _ptr(x2), c2, n_samples, rows_per_sample,
+    fn = N.load().hi3d_groupnorm_silu_det if det else N.load().hi3d_groupnorm_silu
+    N.check(fn(x1.data_ptr(), x1.shape[-1], _ptr(x2), c2, n_samples, rows_per_sample,
                                          gamma.data_ptr(), beta.data_ptr(), eps, int(silu), y.data_ptr(),
                                          ws.data_ptr(), _stream()), "hi3d_groupnorm_silu")
 
 
 def groupnorm_sums(x1: torch.Tensor, x2: Optional[torch.Tensor], n_samples: int, rows_per_sample: int, sums: torch.Tensor,
-                   ws: torch.Tensor):
+                   ws: torch.Tensor, det: bool = False):
     """Local (sum, sumsq) per (sample, group) -> sums fp32 [n_samples, 32, 2] (all-reduced by the caller when sharded)."""
     _chk16(x1, "x1"); _chk32(sums, "sums")
     c2 = 0 if x2 is None else x2.shape[-1]
-    N.check(N.load().hi3d_groupnorm_sums(x1.data_ptr(), x1.shape[-1], _ptr(x2), c2, n_samples, rows_per_sample,
+    fn = N.load().hi3d_groupnorm_sums_det if det else N.load().hi3d_groupnorm_sums
+    N.check(fn(x1.data_ptr(), x1.shape[-1], _ptr(x2), c2, n_samples, rows_per_sample,
                                          sums.data_ptr(), ws.data_ptr(), _stream()), "hi3d_groupnorm_sums")
 
 
@@ -188,17 +206,31 @@ def groupnorm_apply_stats(x1: torch.Tensor, stats1: torch.Tensor, x2: Optional[t
                                                 y_next, frame_rows, _stream()), "hi3d_groupnorm_apply_stats")
 
 
-def groupnorm_unit_stats(x: torch.Tensor, n_images: int, rows_per_image: int, unit: int, stats: torch.Tensor):
+def groupnorm_unit_stats(x: torch.Tensor, n_images: int, rows_per_image: int, unit: int, stats: torch.Tensor,
+                         partials: Optional[torch.Tensor] = None):
+    """Unit table of x, accumulated into `stats`; with `partials` (scratch) deterministic, and `stats` is overwritten."""
     _chk16(x, "x"); _chk32(stats, "stats")
+    if partials is not None:
+        _chk32(partials, "partials")
+        N.check(N.load().hi3d_groupnorm_unit_stats_det(x.data_ptr(), x.shape[-1], n_images, rows_per_image, unit, stats.data_ptr(),
+                                                       partials.data_ptr(), partials.numel(), _stream()),
+                "hi3d_groupnorm_unit_stats_det")
+        return
     N.check(N.load().hi3d_groupnorm_unit_stats(x.data_ptr(), x.shape[-1], n_images, rows_per_image, unit, stats.data_ptr(),
                                                _stream()), "hi3d_groupnorm_unit_stats")
 
 
 def groupnorm_group_sums(stats1: torch.Tensor, C1: int, stats2: Optional[torch.Tensor], C2: int, unit: int, n_samples: int,
-                         imgs_per_sample: int, sums: torch.Tensor):
+                         imgs_per_sample: int, sums: torch.Tensor, det: bool = False):
     _chk32(stats1, "stats1"); _chk32(sums, "sums")
-    N.check(N.load().hi3d_groupnorm_group_sums(stats1.data_ptr(), C1, _ptr(stats2), C2, unit, n_samples, imgs_per_sample,
+    fn = N.load().hi3d_groupnorm_group_sums_det if det else N.load().hi3d_groupnorm_group_sums
+    N.check(fn(stats1.data_ptr(), C1, _ptr(stats2), C2, unit, n_samples, imgs_per_sample,
                                                sums.data_ptr(), _stream()), "hi3d_groupnorm_group_sums")
+
+
+def groupnorm_partials_floats(n_images: int, rows_per_image: int, C: int, unit: int) -> int:
+    """Scratch floats a deterministic producer of an [n_images, C / unit, 2] statistics table needs."""
+    return int(N.load().hi3d_groupnorm_partials_floats(n_images, rows_per_image, C, unit))
 
 
 def layernorm(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, y: torch.Tensor, M: int,

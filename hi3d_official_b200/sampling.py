@@ -363,8 +363,8 @@ class BaseDiffusionSampler:
         if x.shape[0] % T:
             return None
         F_, _, H, W = x.shape
-        key = (id(unet), F_, H, W, T, unet.engine, shard)
-        pkey = (2 * F_, H, W, T, unet.engine) if shard is None else (2 * F_, H, W, T, unet.engine, shard)
+        pkey = unet.plan_key(2 * F_, H, W, T, shard)       # holds the engine and the deterministic-mode switch
+        key = (id(unet),) + pkey
         st = self._fused.get(key)
         if st is None or st.plan is not unet._plans.get(pkey):
             st = self._fused[key] = _FusedState(unet, F_, H, W, T, scale, shard)

@@ -233,12 +233,18 @@ class VideoUNet(nn.Module):
         return P
 
     # ---- plans --------------------------------------------------------------------------------------------
+    def plan_key(self, N: int, H: int, W: int, T: int, shard: Optional[Tuple[int, int]] = None) -> tuple:
+        """Key of the launch plan get_plan returns now: the shape, the engine and the deterministic-mode switch
+        (ops.deterministic(), read here), so that toggling the switch builds a fresh plan instead of replaying a stale one."""
+        key = (N, H, W, T, self.engine, ops.deterministic())
+        return key if shard is None else key + (tuple(shard),)
+
     def get_plan(self, N: int, H: int, W: int, T: int, shard: Optional[Tuple[int, int]] = None) -> "_Plan":
         """shard = (rank, world): frame-sharded plan -- N = B * T local samples, this rank owns frames
         [rank*T, (rank+1)*T) of clips of world*T frames (SURVEY 8e; needs an initialised torch.distributed group)."""
-        key = (N, H, W, T, self.engine) if shard is None else (N, H, W, T, self.engine, tuple(shard))
+        key = self.plan_key(N, H, W, T, shard)
         if key not in self._plans:
-            self._plans[key] = _Plan(self, N, H, W, T, shard=shard)
+            self._plans[key] = _Plan(self, N, H, W, T, shard=shard, det=key[5])
         return self._plans[key]
 
     # ---- reference-compatible forward ------------------------------------------------------------------------
@@ -269,7 +275,9 @@ class VideoUNet(nn.Module):
 class _Plan:
     """Flat launch list for one (N, H, W, T): buffers, pre-baked GEMM parameter blocks, per-step entry points."""
 
-    def __init__(self, net: VideoUNet, N: int, H: int, W: int, T: int, shard: Optional[Tuple[int, int]] = None):
+    def __init__(self, net: VideoUNet, N: int, H: int, W: int, T: int, shard: Optional[Tuple[int, int]] = None,
+                 det: bool = False):
+        self.det = det                 # deterministic GroupNorm statistics (ops.deterministic())
         self.shard = None if shard is None or shard[1] == 1 else (int(shard[0]), int(shard[1]))
         self.rank, self.world = self.shard if self.shard else (0, 1)
         self.Tg = T * self.world                     # frames per clip over all ranks
@@ -322,6 +330,9 @@ class _Plan:
                          and net.cfg.model_channels * max(net.cfg.channel_mult) // self.gn_unit <= 256)
         self._stats_floats = 0
         self.stats_arena = None
+        # deterministic mode: scratch for the statistics partials, shared by every producer (a table is dead once folded)
+        self._part_floats = 0
+        self.gn_part = None
         self._nvtx_open = False
         self.steps: List = []          # main per-step launch list (built lazily as (kind, builder) then baked)
         self._build: List = []         # deferred builders, run after the arena is materialised
@@ -367,15 +378,19 @@ class _Plan:
         """Defer Gemm construction until buffers exist. segs_fn() -> list[SegSpec]; tensor kwargs may be LazyBuf.
         gn_defer: the caller adds the separate statistics pass itself (several launches fill one tensor)."""
         post = None
+        if kw.get("gn_stats") is not None:
+            self._need_partials(kw["gn_stats"], out)
         if kw.get("gn_stats") is not None and W.shape[1] < self.GN_FUSE_MIN_K:
             st, unit, rows = kw.pop("gn_stats"), kw.pop("gn_unit"), kw.pop("gn_rows")
             if not gn_defer:
-                post = lambda: (lambda: ops.groupnorm_unit_stats(out.t, st.n_img, (out.rows // st.n_img), unit, st.t))
+                post = lambda: (lambda: ops.groupnorm_unit_stats(out.t, st.n_img, (out.rows // st.n_img), unit, st.t, self.gn_part))
 
         def build():
             k2 = {}
             for k, v in kw.items():
                 k2[k] = v.t if isinstance(v, (LazyBuf, StatsBuf)) else v
+            if self.det and "gn_stats" in k2:
+                k2["gn_partials"] = self.gn_part
             g = ops.Gemm(segs_fn(), W, out.t if isinstance(out, LazyBuf) else out, M, engine=self.engine, **k2)
             self.flops += g.flops if lst is self._build else 0.0
             return g
@@ -395,6 +410,12 @@ class _Plan:
                 torch.cuda.nvtx.range_push(name)
                 self._nvtx_open = True
             self._call(self._build, m, kind="marker")
+
+    def _need_partials(self, st: StatsBuf, out: LazyBuf):
+        """Deterministic mode: grow the partials scratch to what the producer of `st` (over the tensor `out`) needs."""
+        if self.det:
+            self._part_floats = max(self._part_floats, ops.groupnorm_partials_floats(st.n_img, out.rows // st.n_img, out.cols,
+                                                                                     self.gn_unit))
 
     def _stats(self, n_img: int, C: int) -> Optional[StatsBuf]:
         if not self.gn_fused:
@@ -424,7 +445,7 @@ class _Plan:
         else:
             assert not halo and count_rows is None
             self._call(lst, lambda: ops.groupnorm_silu(x1.t, x2.t if x2 else None, n_samples, rows_per_sample, gam, bet, eps,
-                                                       silu, y.t, ws), kind="groupnorm", bytes=6.0 * M * C)
+                                                       silu, y.t, ws, self.det), kind="groupnorm", bytes=6.0 * M * C)
 
     def _call(self, lst, fn, **meta):
         """meta: kind / flops / bytes = algorithmic work of the launch (read by bench.py's breakdown)."""
@@ -522,6 +543,8 @@ class _Plan:
         A.materialise()
         if self.gn_fused:
             self.stats_arena = torch.zeros(max(self._stats_floats, 2), dtype=torch.float32, device=self.dev)
+        if self.det:
+            self.gn_part = torch.empty(max(self._part_floats, 4), dtype=torch.float32, device=self.dev)
         self.steps = [b() for b in self._build]
         self.cond_steps = [b() for b in self._cond_build]
         self._build = self._cond_build = None
@@ -550,7 +573,7 @@ class _Plan:
                        gn_defer=True, **kw)
         if kw.get("gn_stats") is not None and not fused:       # one statistics pass over the tensor the four launches filled
             st, unit = kw["gn_stats"], kw["gn_unit"]
-            self._call(lst, lambda: ops.groupnorm_unit_stats(out.t, st.n_img, out.rows // st.n_img, unit, st.t),
+            self._call(lst, lambda: ops.groupnorm_unit_stats(out.t, st.n_img, out.rows // st.n_img, unit, st.t, self.gn_part),
                        kind="groupnorm", bytes=2.0 * out.rows * out.cols)
 
     def _emb_slice(self, q):
@@ -622,8 +645,8 @@ class _Plan:
             def local_sums(dst_sums, src=src, sst=sst):
                 """this rank's (sum, sumsq) per (clip, group): from the producer's unit table, or a statistics pass"""
                 if sst is not None:
-                    return ops.groupnorm_group_sums(sst.t, cout, None, 0, self.gn_unit, B, T, dst_sums)
-                return ops.groupnorm_sums(src.t, None, B, T * HW, dst_sums, ws)
+                    return ops.groupnorm_group_sums(sst.t, cout, None, 0, self.gn_unit, B, T, dst_sums, self.det)
+                return ops.groupnorm_sums(src.t, None, B, T * HW, dst_sums, ws, self.det)
             if self.peer is not None:
                 # peer memory: partial sums ride on the exchange kernel (all-reduce in one launch); the halo frames are
                 # stored into the neighbours' buffers by the apply kernel itself; a second exchange orders those stores
@@ -644,7 +667,7 @@ class _Plan:
                 from . import dist as D
                 self._call(bl, lambda ls=local_sums: ls(self.gn_sums), kind="groupnorm",
                            bytes=0.0 if sst is not None else 2.0 * M * cout)
-                self._call(bl, lambda: D.allreduce_sum_(self.gn_sums), kind="nccl")
+                self._call(bl, lambda: D.allreduce_sum_(self.gn_sums, deterministic=self.det), kind="nccl")
                 self._call(bl, lambda src=src, gg=gg, bb=bb: ops.groupnorm_apply(
                     src.t, None, B, T * HW, self.gn_sums, self.Tg * HW, gg, bb, 1e-5, True, gh.t, (T + 2) * HW, HW),
                     kind="groupnorm", bytes=4.0 * M * cout)

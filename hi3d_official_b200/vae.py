@@ -29,8 +29,11 @@ COUT_PAD = 8
 class _VAEPlan:
     """Launch plan for encoder or decoder at one (n, H, W)."""
 
-    def __init__(self, ae: "AutoencoderKL", which: str, n: int, H: int, W: int, T: int = 0):
+    def __init__(self, ae: "AutoencoderKL", which: str, n: int, H: int, W: int, T: int = 0, det: bool = False):
         self.ae, self.which, self.n, self.H, self.W, self.T = ae, which, n, H, W, T
+        self.det = det                 # deterministic GroupNorm statistics (ops.deterministic())
+        self._part_floats = 0          # deterministic mode: partials scratch shared by every statistics producer
+        self.gn_part = None
         self.P = ae._pack()
         self.dev = ae.device
         self.A = Arena(self.dev)
@@ -56,6 +59,8 @@ class _VAEPlan:
         self.A.materialise()
         if self.gn_fused:
             self.stats_arena = torch.zeros(max(self._stats_floats, 2), dtype=torch.float32, device=self.dev)
+        if self.det:
+            self.gn_part = torch.empty(max(self._part_floats, 4), dtype=torch.float32, device=self.dev)
         self.steps = [b() for b in self._build]
         self._build = None
 
@@ -65,6 +70,8 @@ class _VAEPlan:
             def res(v):
                 return v.t if isinstance(v, (LazyBuf, StatsBuf)) else (v() if callable(v) else v)
             k2 = {k: res(v) for k, v in kw.items()}
+            if self.det and "gn_stats" in k2:
+                k2["gn_partials"] = self.gn_part
             g = ops.Gemm(segs_fn(), res(W), res(out), M, engine=self.ae.engine, **k2)
             self.flops += g.flops
             return g
@@ -81,6 +88,8 @@ class _VAEPlan:
         sb = StatsBuf(self, self._stats_floats, self.n, C // self.gn_unit)
         self._stats_floats += self.n * (C // self.gn_unit) * 2
         self._last_stats[(out.tag, out.rows, out.cols)] = sb
+        if self.det:
+            self._part_floats = max(self._part_floats, ops.groupnorm_partials_floats(self.n, out.rows // self.n, C, self.gn_unit))
         return dict(gn_stats=sb, gn_unit=self.gn_unit, gn_rows=rows_per_img)
 
     def _nxt(self, rows, C):
@@ -96,7 +105,7 @@ class _VAEPlan:
             self._call(lambda: ops.groupnorm_apply_stats(x.t, st.t, None, None, self.gn_unit, ns, rows, ips, rows, g, b, eps,
                                                          silu, y.t))
         else:
-            self._call(lambda: ops.groupnorm_silu(x.t, None, ns, rows, g, b, eps, silu, y.t, self.gn_ws))
+            self._call(lambda: ops.groupnorm_silu(x.t, None, ns, rows, g, b, eps, silu, y.t, self.gn_ws, self.det))
 
     def _conv(self, src: LazyBuf, key: str, out: LazyBuf, ho, wo, hs, ws, stride=1, ups=0, pad_lo=1, **kw):
         Wt, b = self.P[key]
@@ -400,9 +409,9 @@ class AutoencoderKL(nn.Module):
         return P
 
     def _plan(self, which: str, n: int, H: int, W: int, T: int = 0) -> _VAEPlan:
-        key = (which, n, H, W, self.engine, T)
+        key = (which, n, H, W, self.engine, T, ops.deterministic())
         if key not in self._plans:
-            self._plans[key] = _VAEPlan(self, which, n, H, W, T)
+            self._plans[key] = _VAEPlan(self, which, n, H, W, T, det=key[-1])
         return self._plans[key]
 
     # -- reference API --------------------------------------------------------------------------------------------------

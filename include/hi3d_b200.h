@@ -114,6 +114,22 @@ int hi3d_gemm_tc5(const hi3d_gemm_params* p, void* stream);
  * HI3D_TC5_PAIR at first use), 0 = always single CTA, 1 = always CTA pairs.  Process-wide; the parity tests run every
  * geometry under both settings (no reference counterpart: the reference's cuDNN / cuBLAS pick their own tiles). */
 int hi3d_gemm_tc5_set_pair_mode(int mode);
+/* Deterministic GroupNorm statistics: hi3d_gemm / hi3d_gemm_tc5 with p->gn_stats produced without float atomics, in an order
+ * that depends on the shapes and the tile geometry only, so that the same inputs give the same bits on every run.  gn_stats is
+ * OVERWRITTEN (no zeroing needed).  `partials` is caller-owned fp32 scratch of partials_floats >=
+ * hi3d_groupnorm_partials_floats(n_images, output rows per image, N, gn_unit) floats; it is dead once the statistics are
+ * complete and may be reused by the next producer on the same stream.  How the table is produced:
+ *   - hi3d_gemm_tc5_det, specialised GroupNorm epilogues, gn_unit == 4 or >= 8, and every 32-row warp block inside one image
+ *     (PLAIN: gn_rows % 32 == 0; CONV2D: tile patch of >= 32 pixels per image; TEMPORAL: >= 32 pixels per frame): each
+ *     epilogue warp STORES its per-octet partials into its own slot (one slot per image, 32-row block and 8-channel octet;
+ *     the four parity-class launches of an up-conv have separate slots) and hi3d_groupnorm_fold sums them after the launch
+ *     (after the out_py = out_px = 1 launch of an up-conv);
+ *   - otherwise (narrower units, several images inside a warp -- test-sized models only -- the generic epilogue, or the
+ *     mma.sync engine) the GEMM runs without epilogue statistics and hi3d_groupnorm_unit_stats_det reads the stored tensor
+ *     (after the last parity launch of an up-conv; out_ld must equal N).
+ * Without gn_stats they are hi3d_gemm / hi3d_gemm_tc5. */
+int hi3d_gemm_det(const hi3d_gemm_params* p, float* partials, int64_t partials_floats, void* stream);
+int hi3d_gemm_tc5_det(const hi3d_gemm_params* p, float* partials, int64_t partials_floats, void* stream);
 /* Test / tuning hook: epilogue warps of the specialised bias-only and GEGLU epilogues: -1 = automatic (16 when K <= 640, the
  * GEMMs whose epilogue is the bound), 8 or 16 forced.  Process-wide; default from HI3D_TC5_EW. */
 int hi3d_gemm_tc5_set_epilogue_warps(int warps);
@@ -172,6 +188,33 @@ int hi3d_groupnorm_apply_halo(const void* x1, int C1, const void* x2, int C2, in
                               const float* sums, int64_t count_rows, const float* gamma, const float* beta, float eps,
                               int apply_silu, void* y, int64_t y_sample_rows, int64_t y_row_off, void* y_prev_rank,
                               void* y_next_rank, int64_t frame_rows, void* stream);
+
+/* Deterministic GroupNorm statistics: the same contracts without float atomics, every sum in an order fixed by the shapes
+ * (and launch geometry) alone, so the same inputs give bit-identical results run after run.  They are what a launch plan
+ * uses when torch.use_deterministic_algorithms(True) or HI3D_DETERMINISTIC=1 is in effect.  Bit-identity holds for one
+ * build on one GPU type and one configuration; a different tile geometry, engine or sharding may round differently.
+ *   hi3d_groupnorm_silu_det / hi3d_groupnorm_sums_det: as hi3d_groupnorm_silu / _sums (same workspace).
+ *   hi3d_groupnorm_group_sums_det: as hi3d_groupnorm_group_sums.
+ *   hi3d_groupnorm_unit_stats_det: the unit table of x, OVERWRITTEN (not accumulated): one partials slot per (image, chunk),
+ *     stored by the statistics pass, then hi3d_groupnorm_fold.  `partials` = fp32 scratch of partials_floats >=
+ *     hi3d_groupnorm_partials_floats(n_images, rows_per_image, C, unit) floats.
+ *   hi3d_groupnorm_partials_floats: scratch floats any deterministic producer of an [n_images, C / unit, 2] table over
+ *     rows_per_image output rows per image needs (0 on bad arguments).
+ *   hi3d_groupnorm_fold: stats[n, u, :] = sum over the blocks_per_image slots of image n of a partials table, in fp64, in a
+ *     fixed order, stored as fp32 (overwrites stats).  octets = 0: slots [n_images, blocks_per_image, C / unit, 2] (the
+ *     statistics pass); octets = 1: slots [n_images, blocks_per_image, C / 8, 4] = (sum, sumsq) of the first unit an
+ *     8-channel octet touches, then of the next one (the tc5 epilogue; unit == 4 or >= 8). */
+int hi3d_groupnorm_silu_det(const void* x1, int C1, const void* x2, int C2, int n_samples, int64_t rows_per_sample,
+                            const float* gamma, const float* beta, float eps, int apply_silu, void* y, float* ws, void* stream);
+int hi3d_groupnorm_sums_det(const void* x1, int C1, const void* x2, int C2, int n_samples, int64_t rows_per_sample, float* sums,
+                            float* ws, void* stream);
+int hi3d_groupnorm_group_sums_det(const float* stats1, int C1, const float* stats2, int C2, int unit, int n_samples,
+                                  int imgs_per_sample, float* sums, void* stream);
+int hi3d_groupnorm_unit_stats_det(const void* x, int C, int n_images, int64_t rows_per_image, int unit, float* stats,
+                                  float* partials, int64_t partials_floats, void* stream);
+int64_t hi3d_groupnorm_partials_floats(int n_images, int64_t rows_per_image, int C, int unit);
+int hi3d_groupnorm_fold(const float* partials, int n_images, int blocks_per_image, int octets, int C, int unit, float* stats,
+                        void* stream);
 
 /* LayerNorm over the last dim C (<= 2560, multiple of 8) of [M, C] fp16 (+ optional broadcast add before the norm:
  * x + addvec[((m / add_div) % add_mod), :], the `x_mix = x + emb` of video_attention.py:286-287).

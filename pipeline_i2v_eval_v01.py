@@ -102,6 +102,14 @@ def cond_from_towers(model, frames, towers, elevation, stage):
     return c, uc
 
 
+def enable_deterministic():
+    """--deterministic: the same seed and inputs give bit-identical frames (same GPU type, build and configuration).  Set
+    before CUDA is initialised, so that cuBLAS in the torch-side conditioner is covered too; the engine's launch plans
+    then use the deterministic GroupNorm statistics (hi3d_official_b200.ops.deterministic)."""
+    os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")
+    torch.use_deterministic_algorithms(True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--denoise_config", type=str, default="configs/inference-v01.yaml")
@@ -114,7 +122,10 @@ def main():
     ap.add_argument("--synthetic", action="store_true")
     ap.add_argument("--tiny", action="store_true")
     ap.add_argument("--seed", type=int, default=None)
+    ap.add_argument("--deterministic", action="store_true", help="bit-identical output for the same seed and inputs")
     params = ap.parse_args()
+    if params.deterministic:
+        enable_deterministic()
     seed = random.randint(0, 65535) if params.seed is None else params.seed      # v01:33-34
     torch.manual_seed(seed)
     model = load_model(params.denoise_config, params.denoise_checkpoint, 1, params.tiny)

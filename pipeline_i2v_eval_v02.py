@@ -12,7 +12,7 @@ import random
 import torch
 import torch.nn.functional as F
 
-from pipeline_i2v_eval_v01 import cond_from_towers, load_model, save_frames, synthetic_cond
+from pipeline_i2v_eval_v01 import cond_from_towers, enable_deterministic, load_model, save_frames, synthetic_cond
 
 
 def main():
@@ -27,7 +27,10 @@ def main():
     ap.add_argument("--synthetic", action="store_true")
     ap.add_argument("--tiny", action="store_true")
     ap.add_argument("--seed", type=int, default=None)
+    ap.add_argument("--deterministic", action="store_true", help="bit-identical output for the same seed and inputs")
     params = ap.parse_args()
+    if params.deterministic:
+        enable_deterministic()
     seed = random.randint(0, 65535) if params.seed is None else params.seed
     torch.manual_seed(seed)
     model = load_model(params.denoise_config, params.denoise_checkpoint, 2, params.tiny)
